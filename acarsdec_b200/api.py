@@ -493,8 +493,9 @@ class Context:
                 out.append(None)
         return out
 
-    def read_dm(self, nsamp: int) -> np.ndarray:
-        out = np.empty((self.nstreams, nsamp, self.nch), dtype=np.float32)
+    def read_dm(self, nsamp: int, streams: int | None = None) -> np.ndarray:
+        """Envelope of the last submit, (streams, nsamp, nch): all streams, or the first `streams`."""
+        out = np.empty((self.nstreams if streams is None else streams, nsamp, self.nch), dtype=np.float32)
         _check(self.lib, self.lib.acb_read_dm(self.h, out.ctypes.data, out.size))
         return out
 

@@ -59,8 +59,11 @@ def _run(cmd, log: Path) -> None:
 def build(force: bool = False, verbose: bool = False) -> Path:
     """Build what is stale.  Several processes may call this at once (one rank per GPU under torchrun): an
     exclusive file lock serialises them, each link goes to a temporary name and is renamed into place, and
-    whoever gets the lock second finds everything up to date."""
+    whoever gets the lock second finds everything up to date.  A tree that is up to date is only read (it may be
+    read-only)."""
     import fcntl
+    if not force and not _lib_stale() and not _compat_stale():
+        return LIB
     (PKG / "build").mkdir(exist_ok=True)
     with open(PKG / "build" / ".lock", "w") as lock:
         fcntl.flock(lock, fcntl.LOCK_EX)
@@ -78,14 +81,21 @@ def _link(cmd, target: Path, log: Path) -> None:
     os.replace(tmp, target)
 
 
+def _lib_stale() -> bool:
+    return _stale(LIB, LIB_SRC + HEADERS + [Path(__file__)])
+
+
+def _compat_stale() -> bool:
+    return all(p.exists() for p in COMPAT_SRC) and any(_stale(t, COMPAT_SRC + HEADERS + [LIB]) for _, t in COMPAT_VARIANTS)
+
+
 def _build_locked(force: bool, verbose: bool) -> Path:
-    if force or _stale(LIB, LIB_SRC + HEADERS + [Path(__file__)]):
+    if force or _lib_stale():
         cmd = [nvcc(), *ARCH, *NVCC_FLAGS, "-shared", "-o", LIB, *LIB_SRC, "-I", ROOT / "include"]
         _link(cmd, LIB, PKG / "build" / "libacars_b200.log")
         if verbose:
             print((PKG / "build" / "libacars_b200.log").read_text())
-    if all(p.exists() for p in COMPAT_SRC) and (
-            force or any(_stale(t, COMPAT_SRC + HEADERS + [LIB]) for _, t in COMPAT_VARIANTS)):
+    if all(p.exists() for p in COMPAT_SRC) and (force or _compat_stale()):
         # plain C, the reference's language; the host's WITH_* macro selects channel_t's layout
         # (acarsdec.h:62-74) and the front-end symbols, so there is one shim per front-end
         for macro, target in COMPAT_VARIANTS:

@@ -77,6 +77,10 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-alt", action="store_true", help="skip the measurement of the other channelizer form")
     ap.add_argument("--no-check", action="store_true", help="skip the oracle check of the timed frames")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed for the distinct pool streams as DIR/*.npy "
+                         "(envelope, decoded frames); the stream count is then --streams, or %d without the sweep, so that "
+                         "the same arguments give the same inputs" % SWEEP[-1])
     ap.add_argument("--cpu-worker", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--variant", default="", help=argparse.SUPPRESS)
     ap.add_argument("--worker-blocks", type=int, default=256, help=argparse.SUPPRESS)
@@ -239,6 +243,22 @@ def check_frames(K: int, pool, reps: int, recs, exact: bool, nstreams: int, per_
     if not exact:
         out["note"] = "messages (chn, len, err, text, BCS) identical; lvl within 0.05 dB (fast channelizer)"
     return out
+
+
+def dump_outputs(d: str, m: dict, B: int) -> None:
+    """The timed path's results in its last step (pass m["passes"]) for the distinct pool streams, which every other
+    stream repeats: envelope.npy float32 (stream, sample, channel); frames.npy float64, one row per decoded frame in
+    emission order (stream, chn, len, err, lvl, block, pos, soh_pos, crc[0], crc[1]); frames_txt.npy float32, the
+    frames' text bytes, zero past len."""
+    d = Path(d)
+    d.mkdir(parents=True, exist_ok=True)
+    recs = m["recs"][m["recs"]["block"] >= (m["passes"] - 1) * B]
+    cols = [recs[f].astype(np.float64) for f in ("stream", "chn", "len", "err", "lvl", "block", "pos", "soh_pos")]
+    np.save(d / "envelope.npy", m["dm_last"])
+    np.save(d / "frames.npy", np.stack(cols + [recs["crc"][:, 0].astype(np.float64), recs["crc"][:, 1].astype(np.float64)], axis=1))
+    txt = recs["txt"].astype(np.float32)
+    txt[np.arange(txt.shape[1])[None, :] >= recs["len"][:, None]] = 0
+    np.save(d / "frames_txt.npy", txt)
 
 
 def rec_tuple(m):
@@ -455,6 +475,8 @@ def main():
     sweep = None
     if args.streams > 0:
         S = args.streams
+    elif args.dump_outputs:
+        S = SWEEP[-1]
     else:
         sweep = []
         for Ssw in SWEEP:
@@ -484,7 +506,7 @@ def main():
     pool_b = [p[:stride] for p in pool]
     samples_per_step_rank = S * B * 1024 * K
 
-    def measure(channelizer: str, steps: int, warmup: int, with_e2e: bool, clk=None):
+    def measure(channelizer: str, steps: int, warmup: int, with_e2e: bool, clk=None, dump: bool = False):
         """One context at (S, B): first pass through the host API from reset state, `warmup` + `steps` device-resident
         submits (timed with the library's CUDA events), an isolated-kernel pass, optionally the host-buffer leg."""
         out = {}
@@ -552,6 +574,8 @@ def main():
         out["per_stream"] = per_stream
         out["passes"] = 1 + warmup + steps
         out["frames_timed"] = int(sum(nframes[n_before:]))
+        if dump:
+            out["dm_last"] = ctx.read_dm(B * 1024, streams=len(pool_b))
         # isolated kernels: sync between steps, so nothing overlaps
         for _ in range(3):
             ctx.submit_device(din.ptr, B, stride)
@@ -589,7 +613,9 @@ def main():
         return out
 
     clk = ClockSampler(local)
-    main_m = measure(args.channelizer, args.steps, args.warmup, not args.no_e2e, clk)
+    main_m = measure(args.channelizer, args.steps, args.warmup, not args.no_e2e, clk, dump=bool(args.dump_outputs) and rank == 0)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, main_m, B)
     clocks = clk.summary(main_m["t0"], main_m["t1"])
     clk.stop()
     total_samples = sum_over_ranks(float(samples_per_step_rank * args.steps))

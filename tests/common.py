@@ -39,6 +39,11 @@ def state_tuple_from_json(j):
 
 
 def bits_equal(a: np.ndarray, b: np.ndarray) -> bool:
+    from refs import Digest
+    if isinstance(b, Digest):
+        a, b = b, a
+    if isinstance(a, Digest):
+        return a == b                                    # a recorded reference array: same shape and float32 bits
     a = np.ascontiguousarray(a, dtype=np.float32)
     b = np.ascontiguousarray(b, dtype=np.float32)
     return a.shape == b.shape and np.array_equal(a.view(np.uint32), b.view(np.uint32))

@@ -54,15 +54,12 @@ def oracle():
 
 
 @pytest.fixture()
-def reflib():
-    """The unmodified reference compiled in place (process-global state: one user at a time)."""
+def reflib(request):
+    """The unmodified reference compiled in place, as recorded for this test (refs.Recorded; process-global state
+    when live: one user at a time)."""
     import refs
-    refs.ensure_built()
-    if not refs.ref_available("O2"):
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
-    r = refs.RefLib("O2")
-    yield r
-    r.close()
+    with refs.recorded(request, lambda: refs.RefLib("O2")) as r:
+        yield r
 
 
 @pytest.fixture(scope="session")

@@ -4,11 +4,17 @@ RefLib    — oracle/_ref/libacarsref_*.so: the unmodified reference compiled in
             It is process-global (the reference keeps its state in globals), so one
             instance at a time per process.
 OracleLib — oracle/libacars_oracle.so: the re-entrant C restatement.
+Recorded  — what the reference returned in one test, replayed from tests/golden/reference/.
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes as C
+import gzip
+import hashlib
+import json
 import os
+import re
 import subprocess
 from pathlib import Path
 
@@ -16,6 +22,8 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent.parent
 ORACLE_DIR = ROOT / "oracle"
+RECORDINGS = ROOT / "tests" / "golden" / "reference"
+RECORD = os.environ.get("ACB_RECORD_REFERENCE") == "1"
 
 
 def ensure_built() -> None:
@@ -517,6 +525,216 @@ class OracleLib:
         out = Msg()
         C.memmove(C.byref(out), C.byref(m), C.sizeof(Msg))
         return out if self.lib.orc_block_fec(C.byref(out)) else None
+
+
+def mask_time(out: bytes) -> bytes:
+    """The program's output with its wall-clock time stamps (text formats, JSON "timestamp") replaced by <time>."""
+    out = re.sub(rb'"timestamp":[0-9.e+]+', b'"timestamp":<time>', out)
+    return re.sub(rb"\d\d/\d\d/\d{4} \d\d:\d\d:\d\d\.\d{3}", b"<time>", out)
+
+
+class RefPrograms:
+    """The programs oracle/Makefile builds from the unmodified reference under oracle/_ref."""
+
+    def outfmt(self, raw: bytes, *argv: str):
+        """ref_outfmt: the reference's output.c / label.c / netout.c fed the records `raw`; one entry per record,
+        what the reference printed (net == "-") or the one datagram it sent, None for nothing."""
+        net = argv[1]
+        r = subprocess.run([str(ORACLE_DIR / "_ref" / "ref_outfmt"), *argv], input=raw, capture_output=True, timeout=120)
+        assert r.returncode == 0, r.stderr
+        out = []
+        for chunk in r.stdout.split(b"\x1e")[1:]:
+            if net == "-":
+                out.append(chunk or None)
+            else:
+                grams = chunk.split(b"\x1d")[1:]
+                assert len(grams) <= 1
+                out.append(grams[0] if grams else None)
+        return out
+
+    def acarsdec_rtl(self, iq: np.ndarray, *argv: str) -> bytes:
+        """stdout of the whole reference program (acarsdec_ref) on the u8 IQ capture `iq` (file-replay librtlsdr),
+        wall-clock time stamps masked (mask_time)."""
+        import tempfile
+        with tempfile.TemporaryDirectory() as d:
+            cap = Path(d) / "cap.iq"
+            iq.tofile(cap)
+            r = subprocess.run([str(ORACLE_DIR / "_ref" / "acarsdec_ref"), *argv], env=dict(os.environ, ACARSDEC_STUB_IQ=str(cap)),
+                               capture_output=True, timeout=120)
+        assert r.returncode == 0, r.stderr
+        return mask_time(r.stdout)
+
+    def abi_layout(self) -> str:
+        """channel_t / msgblk_t offsets and constants as the reference's acarsdec.h defines them (oracle/abi_layout.c)."""
+        return subprocess.run([str(ORACLE_DIR / "_ref" / "abi_layout")], capture_output=True, text=True, check=True).stdout
+
+    def close(self):
+        pass
+
+
+def _canon(v) -> bytes:
+    """The bytes that identify a value the way the tests compare it: float arrays by shape and float32 bit
+    pattern (common.bits_equal), floats exactly with -0.0 folded into 0.0 (== does not tell them apart)."""
+    if isinstance(v, np.ndarray):
+        if v.dtype.kind == "f":
+            return repr(v.shape).encode() + np.ascontiguousarray(v, dtype=np.float32).tobytes()
+        return v.dtype.str.encode() + repr(v.shape).encode() + np.ascontiguousarray(v).tobytes()
+    if isinstance(v, (bytes, bytearray)):
+        return b"b" + bytes(v)
+    if isinstance(v, (float, np.floating)):
+        return (float(v) + 0.0).hex().encode()
+    if isinstance(v, (tuple, list)):
+        return b"(" + b",".join(_canon(x) for x in v) + b")"
+    if isinstance(v, Path):
+        raise TypeError("a path is not an input of the reference: pass the data")
+    return repr(v).encode()
+
+
+def _digest(v) -> str:
+    return hashlib.sha256(_canon(v)).hexdigest()[:8]
+
+
+class Digest:
+    """A recorded value too large to store: equal to any value with the same _canon bytes (32-bit digest)."""
+    __hash__ = None
+
+    def __init__(self, h: str):
+        self.h = h
+
+    def __eq__(self, other):
+        return self.h == (other.h if isinstance(other, Digest) else _digest(other))
+
+    def __repr__(self):
+        return f"<reference value, digest {self.h}>"
+
+
+class _State:
+    def __init__(self, h: str):
+        self._vec = Digest(h)
+
+    def vec(self):
+        return self._vec
+
+
+def _encode(v):
+    if v is None or isinstance(v, (bool, int, str)):
+        return v
+    if isinstance(v, np.integer):
+        return int(v)
+    if isinstance(v, float):
+        return {"f": v.hex()}
+    if isinstance(v, np.ndarray) and v.dtype.kind in "iu":
+        return {"a": v.dtype.str, "v": v.tolist()}
+    if isinstance(v, (RefState, _State)):
+        return {"state": _digest(v.vec()) if isinstance(v, RefState) else v.vec().h}
+    if isinstance(v, Msg):
+        return {"msg": [v.chn, v.len, v.err, int(np.float32(v.lvl).view(np.uint32)), bytes(v.txt[:v.len]).hex(), bytes(v.crc).hex()]}
+    if isinstance(v, (list, tuple)):
+        return [_encode(x) for x in v]
+    return {"d": _digest(v)}                             # float arrays, bytes
+
+
+def _decode(e):
+    if isinstance(e, list):
+        return [_decode(x) for x in e]
+    if not isinstance(e, dict):
+        return e
+    if "f" in e:
+        return float.fromhex(e["f"])
+    if "a" in e:
+        return np.array(e["v"], dtype=e["a"])
+    if "state" in e:
+        return _State(e["state"])
+    if "msg" in e:
+        chn, ln, err, lvl, txt, crc = e["msg"]
+        m = Msg()
+        m.chn, m.len, m.err = chn, ln, err
+        m.lvl = float(np.uint32(lvl).view(np.float32))
+        m.txt[:ln] = bytes.fromhex(txt)
+        m.crc[:] = bytes.fromhex(crc)
+        return m
+    return Digest(e["d"])
+
+
+class Recorded:
+    """A front-end of the unmodified reference (RefLib, RefAirLib, ...) as one test saw it.
+
+    Replaying, it answers every call with what the reference returned when the recording was made, so the test
+    compares against the reference on a machine that has no reference sources.  Recording (ACB_RECORD_REFERENCE=1,
+    needs oracle/_ref), it forwards to the live library, so the test compares against the reference itself, and
+    writes what it saw.  Calls that only feed the reference (INPUTS) return nothing; every call's name and arguments
+    go into a running hash that each recorded answer carries, so a replay also checks that the test feeds the
+    reference exactly what was recorded.  Numbers, integer tables and messages are stored as they are; float arrays,
+    byte strings and channel states as a Digest."""
+    INPUTS = {"open_rtl", "open_audio", "open", "block", "run", "audio", "push_block", "feed"}
+    ATTRIBUTES = {"fc", "K", "nbch", "which"}
+
+    def __init__(self, path: Path, live=None):
+        self._path, self._live, self._h = path, live, hashlib.sha256()
+        if live is None:
+            if not path.exists():
+                raise FileNotFoundError(f"{path.name}: no recording of the reference for this test "
+                                        "(ACB_RECORD_REFERENCE=1 with oracle/_ref built writes it)")
+            rec = json.loads(gzip.decompress(path.read_bytes()))
+            self._calls, self._end = rec["calls"], rec["end"]
+        else:
+            self._calls, self._end = [], None
+        self._next = 0
+
+    def _answer(self, name: str, args, call):
+        self._h.update(name.encode() + _canon(list(args)))
+        where = self._h.hexdigest()[:8]
+        if self._live is not None:
+            v = call()
+            if name in self.INPUTS:
+                assert v is None, name
+            else:
+                self._calls.append([name, where, _encode(v)])
+            return v
+        if name in self.INPUTS:
+            return None
+        assert self._next < len(self._calls), f"{name}: more calls than recorded"
+        rname, rwhere, v = self._calls[self._next]
+        self._next += 1
+        assert (rname, rwhere) == (name, where), f"call {self._next} ({name}) differs from the recording ({rname}) in name or inputs"
+        return _decode(v)
+
+    def __getattr__(self, name: str):
+        if name.startswith("_"):
+            raise AttributeError(name)
+        if name in self.ATTRIBUTES:
+            return self._answer(name, (), lambda: getattr(self._live, name))
+        return lambda *args: self._answer(name, args, lambda: getattr(self._live, name)(*args))
+
+    def finish(self) -> None:
+        end = self._h.hexdigest()[:8]
+        if self._live is not None:
+            self._path.parent.mkdir(parents=True, exist_ok=True)
+            data = json.dumps({"calls": self._calls, "end": end}, separators=(",", ":")).encode()
+            self._path.write_bytes(gzip.compress(data, 9, mtime=0))
+        else:
+            assert self._next == len(self._calls) and end == self._end, "the test made fewer calls than recorded, or other inputs"
+
+
+@contextlib.contextmanager
+def recorded(request, open_live, close_live=lambda r: r.close()):
+    """Recorded for the running test (tests/golden/reference/<module>.<test>.json.gz); open_live() builds the live
+    front-end when recording."""
+    name = re.sub(r"[^A-Za-z0-9_.-]+", "_", f"{request.node.module.__name__}.{request.node.name}").strip("_")
+    path = RECORDINGS / (name + ".json.gz")
+    live = None
+    if RECORD:
+        ensure_built()
+        live = open_live()
+    r = Recorded(path, live)
+    failed = request.session.testsfailed
+    try:
+        yield r
+        if request.session.testsfailed == failed:       # a failed test neither writes nor checks the rest of the recording
+            r.finish()
+    finally:
+        if live is not None:
+            close_live(live)
 
 
 class Sink:

@@ -9,13 +9,9 @@ from common import bits_equal, msg_tuple
 
 
 @pytest.fixture()
-def airref():
-    refs.ensure_built()
-    if not (refs.ORACLE_DIR / "_ref" / "libacarsref_air_O2.so").exists():
-        pytest.skip("oracle/_ref air build absent")
-    r = refs.RefAirLib()
-    yield r
-    r.close()
+def airref(request):
+    with refs.recorded(request, refs.RefAirLib) as r:
+        yield r
 
 
 @pytest.mark.parametrize("rate,freqs", [

@@ -16,38 +16,21 @@ from common import GOLDEN, load_testwav, msg_tuple, msg_tuple_from_json
 
 ROOT = Path(__file__).resolve().parent.parent
 PKG = ROOT / "acarsdec_b200"
-REF = Path("/root/reference")
 REFBIN = ROOT / "oracle" / "_ref"
 
-LAYOUT_PROG = r'''
-#include <stdio.h>
-#include <stddef.h>
-#include HDR
-#define P(t, f) printf(#t "." #f " %zu\n", offsetof(t, f))
-int main(void) {
-  printf("sizeof(channel_t) %zu\nsizeof(msgblk_t) %zu\n", sizeof(channel_t), sizeof(msgblk_t));
-  P(channel_t, chn); P(channel_t, Fr); P(channel_t, wf); P(channel_t, dm_buffer); P(channel_t, MskPhi); P(channel_t, MskDf);
-  P(channel_t, MskClk); P(channel_t, MskLvlSum); P(channel_t, MskBitCount); P(channel_t, MskS); P(channel_t, idx);
-  P(channel_t, inb); P(channel_t, outbits); P(channel_t, nbits); P(channel_t, Acarsstate); P(channel_t, blk); P(channel_t, th);
-  P(msgblk_t, prev); P(msgblk_t, chn); P(msgblk_t, tv); P(msgblk_t, len); P(msgblk_t, err); P(msgblk_t, lvl); P(msgblk_t, txt); P(msgblk_t, crc);
-  printf("MAXNBCHANNELS %d INTRATE %d WSYN %d END %d\n", MAXNBCHANNELS, INTRATE, (int)WSYN, (int)END);
-  return 0; }
-'''
+
+@pytest.fixture()
+def refprog(request):
+    with refs.recorded(request, refs.RefPrograms) as r:
+        yield r
 
 
-def _run_layout(tmp_path, hdr, incs):
-    src = tmp_path / "l.c"
-    src.write_text(LAYOUT_PROG.replace("HDR", hdr))
-    exe = tmp_path / ("l_" + str(abs(hash(hdr))))
-    subprocess.run(["gcc", "-DWITH_RTL", *incs, "-o", str(exe), str(src)], check=True)
-    return subprocess.run([str(exe)], capture_output=True, text=True, check=True).stdout
-
-
-@pytest.mark.skipif(not REF.exists(), reason="needs the reference tree (build container only)")
-def test_abi_mirror_matches_reference_header(tmp_path):
-    mine = _run_layout(tmp_path, '"acarsdec_compat.h"', ["-I", str(ROOT / "include")])
-    theirs = _run_layout(tmp_path, '"acarsdec.h"', ["-I", str(REF)])
-    assert mine == theirs
+def test_abi_mirror_matches_reference_header(tmp_path, refprog):
+    exe = tmp_path / "abi_layout"
+    subprocess.run(["gcc", "-DWITH_RTL", '-DHDR="acarsdec_compat.h"', "-I", str(ROOT / "include"), "-o", str(exe),
+                    str(ROOT / "oracle" / "abi_layout.c")], check=True)
+    mine = subprocess.run([str(exe)], capture_output=True, text=True, check=True).stdout
+    assert mine == refprog.abi_layout()
 
 
 def _host(tmp_path) -> Path:

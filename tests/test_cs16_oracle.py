@@ -13,12 +13,8 @@ FREQS = (131.525, 131.725, 131.825, 131.450)
 
 @pytest.fixture(params=["soapy", "sdrplay"])
 def cs16ref(request):
-    refs.ensure_built()
-    if not (refs.ORACLE_DIR / "_ref" / f"libacarsref_{request.param}_O2.so").exists():
-        pytest.skip("oracle/_ref CS16 builds absent")
-    r = refs.RefCs16Lib(request.param)
-    yield r
-    r.close()
+    with refs.recorded(request, lambda: refs.RefCs16Lib(request.param)) as r:
+        yield r
 
 
 def test_cs16_plan_tables_carry_and_messages(oracle, cs16ref):

@@ -11,9 +11,6 @@ import pytest
 import refs
 from acarsdec_b200 import api
 
-REFBIN = refs.ORACLE_DIR / "_ref" / "ref_outfmt"
-pytestmark = pytest.mark.skipif(not REFBIN.exists(), reason="oracle/_ref/ref_outfmt absent (needs /root/reference at build time)")
-
 NET = {api.FMT_NET_PP: "N", api.FMT_NET_NATIVE: "n", api.FMT_NET_JSON: "j"}
 
 
@@ -34,26 +31,22 @@ def _records(blocks):
     return raw, msgs
 
 
-def _reference(raw, outtype, net, inmode, airflt, emptymsg, labels, station):
-    r = subprocess.run([str(REFBIN), str(outtype), net, str(inmode), str(int(airflt)), str(int(emptymsg)), labels or "-", station or "-"],
-                       input=raw, capture_output=True, timeout=120)
-    assert r.returncode == 0, r.stderr
-    out = []
-    for chunk in r.stdout.split(b"\x1e")[1:]:
-        if net == "-":
-            out.append(chunk or None)
-        else:
-            grams = chunk.split(b"\x1d")[1:]
-            assert len(grams) <= 1
-            out.append(grams[0] if grams else None)
-    return out
+@pytest.fixture()
+def ref(request):
+    """The reference's programs (refs.RefPrograms) as recorded for this test."""
+    with refs.recorded(request, refs.RefPrograms) as r:
+        yield r
 
 
-def _compare(blocks, *, inmode=3, airflt=False, emptymsg=False, labels=None, station="STA1"):
+def _reference(ref, raw, outtype, net, inmode, airflt, emptymsg, labels, station):
+    return ref.outfmt(raw, str(outtype), net, str(inmode), str(int(airflt)), str(int(emptymsg)), labels or "-", station or "-")
+
+
+def _compare(ref, blocks, *, inmode=3, airflt=False, emptymsg=False, labels=None, station="STA1"):
     raw, msgs = _records(blocks)
     n = 0
     for fmt in (api.FMT_FULL, api.FMT_ONELINE, api.FMT_JSON, api.FMT_NET_PP, api.FMT_NET_NATIVE, api.FMT_NET_JSON):
-        want = _reference(raw, fmt if fmt in (1, 2, 4) else 0, NET.get(fmt, "-"), inmode, airflt, emptymsg, labels, station)
+        want = _reference(ref, raw, fmt if fmt in (1, 2, 4) else 0, NET.get(fmt, "-"), inmode, airflt, emptymsg, labels, station)
         assert len(want) == len(msgs)
         for i, (b, m) in enumerate(zip(blocks, msgs)):
             got = api.format_msg(m, fmt, tv_sec=b[5], tv_usec=b[6], freq_hz=b[1], inmode=inmode, airflt=airflt, emptymsg=emptymsg,
@@ -82,7 +75,7 @@ RULE_TEXTS = {
 }
 
 
-def test_every_label_rule_and_its_near_miss():
+def test_every_label_rule_and_its_near_miss(ref):
     blocks = []
     pad = b" " * 24                       # long enough that no rule reads past the text (undefined in the reference)
     for i, (lab, txt) in enumerate(sorted(RULE_TEXTS.items())):
@@ -91,10 +84,10 @@ def test_every_label_rule_and_its_near_miss():
         miss = bytearray(txt + pad)
         miss[min(4, len(txt) - 1)] ^= 0x01   # disturb a byte most rules guard on or copy
         blocks.append((1, 131725000, _block(label=lab, bid=b"B", text=bytes(miss)), -7.25, 0, T0, 999999))
-    assert _compare(blocks) > 500
+    assert _compare(ref, blocks) > 500
 
 
-def test_header_variants_filters_and_escapes():
+def test_header_variants_filters_and_escapes(ref):
     b = []
     b.append((0, 131525000, _block(text=b'HELLO "WORLD" \\ back\r\nLINE2\ttab\x01\x1f', end=b"\x17"), -12.34, 1, T0, 123456))   # JSON escapes, ETB
     b.append((3, 131825000, _block(ack=b"A", label=b"_\x7f", bid=b"\0", stx=b"\x03", text=b"", no=b"", fid=b""), -3.0, 0, T0, 0))      # squitter, empty
@@ -103,14 +96,14 @@ def test_header_variants_filters_and_escapes():
     b.append((1, 131550000, _block(bid=b"Z", text=b"x" * 200), 9.96, 0, 1, 1))                                                        # long uplink text
     b.append((4, 131725000, _block(label=b"H1", bid=b"2", text=b"A\nB\rC" + b"y" * 80), -20.05, 2, T0, 500))                          # one-line cut at 59
     for inmode in (0, 2, 3, 5):
-        assert _compare(b, inmode=inmode) > 20
-    assert _compare(b, airflt=True) > 10                     # -A: uplinks dropped
-    assert _compare(b, emptymsg=True) > 10                   # -e: empty messages dropped
-    assert _compare(b, labels="H1:5Z") > 5                   # -i H1:5Z
-    assert _compare(b, station="") > 20                      # no station id: no "station_id" key
+        assert _compare(ref, b, inmode=inmode) > 20
+    assert _compare(ref, b, airflt=True) > 10                     # -A: uplinks dropped
+    assert _compare(ref, b, emptymsg=True) > 10                   # -e: empty messages dropped
+    assert _compare(ref, b, labels="H1:5Z") > 5                   # -i H1:5Z
+    assert _compare(ref, b, station="") > 20                      # no station id: no "station_id" key
 
 
-def test_random_blocks():
+def test_random_blocks(ref):
     rng = np.random.default_rng(12)
     printable = np.frombuffer(bytes(range(32, 127)), dtype=np.uint8)
     free_labels = [b"H1", b"5Z", b"SA", b"_d", b"B9", b"A0", b"C1", b"Q0", b"QX", b"30", b"4T"]        # no OOOI rule: any text length is defined
@@ -128,7 +121,7 @@ def test_random_blocks():
                               text=txt, no=bytes(rng.choice(printable, 4)), fid=bytes(rng.choice(printable, 6)),
                               end=bytes([int(rng.choice([3, 0x17]))])),
                        float(np.float32(rng.uniform(-45, 5))), int(rng.integers(0, 4)), T0 + int(rng.integers(0, 10**7)), int(rng.integers(0, 10**6))))
-    assert _compare(blocks) > 8000
+    assert _compare(ref, blocks) > 8000
 
 
 def test_field_split_api():
@@ -146,25 +139,18 @@ def test_field_split_api():
         api.format_msg(m, api.FMT_JSON)
 
 
-@pytest.mark.skipif(not (refs.ORACLE_DIR / "_ref" / "acarsdec_ref").exists(), reason="oracle/_ref/acarsdec_ref absent")
 @pytest.mark.parametrize("outtype,fmt", [("2", api.FMT_FULL), ("1", api.FMT_ONELINE), ("4", api.FMT_JSON)])
-def test_formatter_reproduces_the_reference_programs_stdout(tmp_path, oracle, outtype, fmt):
+def test_formatter_reproduces_the_reference_programs_stdout(oracle, ref, outtype, fmt):
     """End to end on the CPU: the unmodified reference program (its own DSP and its own output.c) on a synthetic capture,
     against the same capture decoded by the restatement and printed by the product's formatter — same stdout, time stamps
     masked (the program stamps wall-clock time)."""
-    import os
-    import re
     from acarsdec_b200 import synth
     K, fm = 160, (131.525, 131.725, 131.825, 131.450, 131.550)
     fd, _, fc = oracle.plan(K, fm)
     plan = synth.make_plan(K, fm, fc, seconds=1.5, seed=123, text_len=(10, 120), msgs_per_chan_per_sec=3.0)
     nblk = synth.blocks_for_seconds(K, 1.5)
     iq = synth.render_blocks(plan, 0, nblk)
-    cap = tmp_path / "cap.iq"
-    iq.tofile(cap)
-    ref = subprocess.run([str(refs.ORACLE_DIR / "_ref" / "acarsdec_ref"), "-o", outtype, "-m", str(K), "-i", "STA1", "-r", "0", *[str(f) for f in fm]],
-                         env=dict(os.environ, ACARSDEC_STUB_IQ=str(cap)), capture_output=True, timeout=120)
-    assert ref.returncode == 0, ref.stderr
+    want = ref.acarsdec_rtl(iq, "-o", outtype, "-m", str(K), "-i", "STA1", "-r", "0", *[str(f) for f in fm])
     o = refs.OracleStream(oracle, K, oracle.wf(K, fm))
     o.blocks(iq.reshape(-1))
     mine = b""
@@ -175,8 +161,7 @@ def test_formatter_reproduces_the_reference_programs_stdout(tmp_path, oracle, ou
         # rtl.c:255 keeps the frequency as int <- float <- unsigned: what channel[].Fr holds and the formats print
         s = api.format_msg(m, fmt, tv_sec=T0, tv_usec=123000, freq_hz=api.load().acb_stored_fr(fd[m.chn]), inmode=3, station_id="STA1")
         mine += s + (b"\n" if fmt == api.FMT_JSON else b"")
-    mask = lambda b: re.sub(rb"\d\d/\d\d/\d{4} \d\d:\d\d:\d\d\.\d{3}", b"<time>", re.sub(rb'"timestamp":[0-9.e+]+', b'"timestamp":<time>', b))
-    assert mask(ref.stdout).count(b"<time>") >= 8 and mask(ref.stdout) == mask(mine)
+    assert refs.mask_time(mine).count(b"<time>") >= 8 and want == refs.mask_time(mine)
 
 
 def _flight_sequence():
@@ -198,10 +183,10 @@ def _flight_sequence():
     return blocks
 
 
-def test_route_json_and_monitor_follow_the_reference_flight_table():
+def test_route_json_and_monitor_follow_the_reference_flight_table(ref):
     blocks = _flight_sequence()
     raw, msgs = _records(blocks)
-    want = _reference(raw, 5, "-", 3, False, False, None, "STA1")              # -o 5: route JSON
+    want = _reference(ref, raw, 5, "-", 3, False, False, None, "STA1")              # -o 5: route JSON
     fl = api.Flights()
     got = [fl.route_json(m, tv_sec=b[5], tv_usec=b[6], station_id="STA1") for b, m in zip(blocks, msgs)]
     got = [g + b"\n" if g else None for g in got]
@@ -215,7 +200,7 @@ def test_route_json_and_monitor_follow_the_reference_flight_table():
     fl.close()
     mixed = blocks[:40] + [(2, 131525000, _block(bid=b"B", label=b"H1", text=b"uplink text"), -5.0, 0, blocks[39][5] + 5, 0)] + blocks[40:]
     raw, msgs = _records(mixed)
-    want = _reference(raw, 3, "-", 3, False, False, None, "STA1")              # -o 3: the monitor screen after every block
+    want = _reference(ref, raw, 3, "-", 3, False, False, None, "STA1")              # -o 3: the monitor screen after every block
     fl = api.Flights()
     got = [fl.monitor(m, 16, tv_sec=b[5], tv_usec=b[6], station_id="STA1") for b, m in zip(mixed, msgs)]
     assert got == want and all(g is not None for g in got)
