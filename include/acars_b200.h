@@ -226,7 +226,11 @@ int acb_submit_cs16_planar_host(acb_ctx_t *ctx, const int16_t *xi, const int16_t
 /* Emission order of the streaming front-ends (SURVEY H5).  The reference runs demodMSK channel by channel on
  * whatever a transfer (air.c:336) or a full dm_buffer (soapy.c:247: 1024 outputs; sdrplay.c:229: 512) delivered, so
  * its messages leave in (group, channel, time) order.  A submit may carry many such groups; tell the context how
- * they are cut and acb_sync / acb_collect queue the frames exactly in the reference's order:
+ * they are cut and acb_sync / acb_collect queue the frames in the reference's order.  A submit boundary always acts
+ * as a group boundary too (a submit's frames are queued when it is collected, never held back for the next one), so
+ * the order is exactly the reference's when every submit ends on a group boundary; a submit that ends inside a
+ * group splits it in two.  A frame belongs to the group holding its completion sample (msg.pos), first and last
+ * samples included:
  *   ACB_GROUP_SUBMIT   one group per submit call (default);
  *   ACB_GROUP_OUTPUTS  a group every `period` envelope samples, counted from the start of the stream;
  *   ACB_GROUP_INPUT    a group per transfer of `period` input samples, counted from the start of the stream.

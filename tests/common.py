@@ -38,6 +38,62 @@ def state_tuple_from_json(j):
             tuple(float.fromhex(x) for x in j["inb"]))
 
 
+def emission_model(oracle, dms, cuts, positions: bool = False):
+    """The reference's loop as a plain model: walk the emission groups; in each, for each stream and each channel in
+    turn, demodMSK on that group's slice of the envelope; then the block FEC.  dms: per stream, a (nch, nout) float32
+    envelope; cuts: the first sample of every group (0 is always one).  Returns the surviving messages in emission
+    order as (stream, msg_tuple, group start, group end, completion sample) and the final channel states
+    [stream][channel].  The completion sample (0-based: the envelope sample whose processing finished the frame) is
+    found by feeding shorter prefixes of the slice to copies of the channel state when `positions` is set, else None."""
+    import ctypes as C
+    import refs
+
+    nout = dms[0].shape[1]
+    bounds = sorted({int(c) for c in cuts if 0 <= c < nout} | {0}) + [nout]
+    chans = [[oracle.new_chan(c) for c in range(d.shape[0])] for d in dms]
+
+    def copy(ch):
+        out = refs.OrcChan()
+        C.memmove(C.byref(out), C.byref(ch), C.sizeof(out))
+        return out
+
+    def count(before, x):
+        sink = refs.Sink()
+        oracle.demod(copy(before), x, sink)
+        return sink.c.nmsg
+
+    out = []
+    for lo, hi in zip(bounds[:-1], bounds[1:]):
+        for s, d in enumerate(dms):
+            for c in range(d.shape[0]):
+                x = np.ascontiguousarray(d[c, lo:hi])
+                before = copy(chans[s][c]) if positions else None
+                sink = refs.Sink()
+                oracle.demod(chans[s][c], x, sink)
+                for i, m in enumerate(sink.msgs()):
+                    p = None
+                    if positions:                        # shortest prefix that yields message i: it completes on its last sample
+                        a, b = 1, len(x)
+                        while a < b:
+                            mid = (a + b) // 2
+                            a, b = (mid + 1, b) if count(before, x[:mid]) <= i else (a, mid)
+                        p = lo + a - 1
+                    f = oracle.fec(m)
+                    if f is not None:
+                        out.append((s, msg_tuple(f), lo, hi, p))
+    return out, chans
+
+
+def assert_emission_order(got, model):
+    """Drained messages (api.Msg, in queue order) against emission_model(): same stream and message at every place,
+    its position inside the group the model put it in, and equal to the model's completion sample where known."""
+    assert [(m.stream, msg_tuple(m)) for m in got] == [(s, t) for s, t, *_ in model]
+    for m, (s, t, lo, hi, p) in zip(got, model):
+        assert lo <= m.pos < hi, (s, t[0], m.pos, lo, hi)
+        if p is not None:
+            assert m.pos == p, (s, t[0], m.pos, p)
+
+
 def bits_equal(a: np.ndarray, b: np.ndarray) -> bool:
     from refs import Digest
     if isinstance(b, Digest):

@@ -320,6 +320,88 @@ def test_demod_every_lane_width(native, oracle, lanes, monkeypatch):
     assert total >= 4
 
 
+def _demod_chunks_vs_oracle(ctx, oracle, dm, chans, chunks):
+    """dm: (nstreams, nsamp, nch) fed through submit_dm in `chunks`; after every chunk the device states must be
+    bit-identical to the oracle's `chans` [stream][chn] fed the same samples, and the chunk's frames identical, in
+    the order (stream, channel, time) one submit queues them.  Returns the number of frames."""
+    nst, nsamp, nch = dm.shape
+    pos = total = 0
+    for n in chunks:
+        if pos >= nsamp:
+            break
+        n = min(n, nsamp - pos)
+        ctx.submit_dm(dm[:, pos:pos + n])
+        ctx.sync()
+        got = [(m.stream, msg_tuple(m)) for m in ctx.drain()]
+        want = []
+        for s in range(nst):
+            for c in range(nch):
+                sink = refs.Sink()
+                oracle.demod(chans[s][c], dm[s, pos:pos + n, c], sink)
+                for m in sink.msgs():
+                    f = oracle.fec(m)
+                    if f is not None:
+                        want.append((s, msg_tuple(f)))
+        pos += n
+        assert got == want, pos
+        for s in range(nst):
+            for c in range(nch):
+                assert ctx.get_state(s, c).vec() == chans[s][c].vec(), (pos, s, c)
+        total += len(want)
+    return total
+
+
+@pytest.mark.parametrize("lanes", [1, 2, 4, 8, 17, 20, 24, 33, 34, 36, 40, -4, -8])
+def test_demod_envelope_extremes_every_lane_width(native, oracle, lanes, monkeypatch):
+    """tests/test_demod_core.py's zero / huge / tiny envelope on the device, where the lanes of a channel's group split
+    the mixer samples: 3000 zeros (lvl = 0: the division guard's slow path), a stretch x1e7, zeros, a stretch x1e-30;
+    2 streams x 11 channels, each chain its own slices, odd chunk sizes.  (Denormal envelopes are left out: the reference
+    is built -Ofast, which flushes them, the oracle is strict IEEE.)"""
+    monkeypatch.setenv("ACB_DEMOD_LANES", str(lanes))
+    K, fm = 160, synth.DEFAULT_FREQS_MHZ
+    _, _, fc = api.plan(K, fm)
+    nblk = synth.blocks_for_seconds(K, 1.0)
+    env = oracle.channelize(synth.render_blocks(synth.make_plan(K, fm, fc, seconds=1.0, seed=21), 0, nblk).reshape(-1), K, oracle.wf(K, fm))
+    nst, nch = 2, 11
+    dm = np.empty((nst, 12000, nch), dtype=np.float32)
+    for s in range(nst):
+        for c in range(nch):
+            a, b, off = env[(s * nch + c) % 8], env[(s * nch + c + 3) % 8], 700 * ((s * nch + c) % 7)
+            dm[s, :, c] = np.concatenate([np.zeros(3000, np.float32), a[off:off + 4000] * np.float32(1e7), np.zeros(2000, np.float32),
+                                          b[off:off + 3000] * np.float32(1e-30)])
+    chans = [[oracle.new_chan(c) for c in range(nch)] for _ in range(nst)]
+    with api.Context(K, nst, nch, 2, flags=1) as ctx:
+        frames = _demod_chunks_vs_oracle(ctx, oracle, dm, chans, [999, 1023, 777, 1, 1501, 2047, 333] * 4)
+    assert frames >= 1
+
+
+@pytest.mark.parametrize("lanes", [1, 2, 4, 8, 24, 40, -4])
+def test_foreign_state_on_the_device(native, oracle, lanes, monkeypatch):
+    """tests/test_demod_core.py's foreign states (bit clock far ahead, big MskDf) set with acb_set_state on every chain:
+    the device follows the reference from there at every lane width."""
+    monkeypatch.setenv("ACB_DEMOD_LANES", str(lanes))
+    x, _ = load_testwav()
+    foreign = [(4.9, 0.0), (7.5, 0.02), (-3.0, -0.03), (0.1, 0.3)]
+    nst, nch = 2, 11
+    dm = np.empty((nst, 9000, nch), dtype=np.float32)
+    chans = [[None] * nch for _ in range(nst)]
+    with api.Context(160, nst, nch, 5, flags=1) as ctx:
+        for s in range(nst):
+            for c in range(nch):
+                i = s * nch + c
+                dm[s, :, c] = x[(i % 3) * 1000:(i % 3) * 1000 + 9000, i % 4]
+                clk, df = foreign[i % 4]
+                st = ctx.get_state(s, c)
+                st.MskClk, st.MskDf = clk, df
+                ctx.set_state(s, c, st)
+                oc = oracle.new_chan(c)
+                oc.MskClk, oc.MskDf = clk, df
+                chans[s][c] = oc
+                assert ctx.get_state(s, c).vec() == oc.vec()
+        frames = _demod_chunks_vs_oracle(ctx, oracle, dm, chans, [1001, 37, 2999, 511, 4452])
+    assert frames >= 1
+
+
 def test_corrupted_frames_fec_on_gpu_path(native, oracle):
     K, fm = 160, (131.525, 131.725, 131.825)
     fd, _, fc = api.plan(K, fm)
