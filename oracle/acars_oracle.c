@@ -456,6 +456,29 @@ void orc_channelize_cs16(int variant, const int16_t *iq, int nout, int K, int nc
 	}
 }
 
+/* A CS16 context with the caller's table (acb_set_wf; taps <= K): the complex MAC of rtl.c:350-352 on (float)int16 with
+ * no bias, product (ac-bd, ad+bc) rounded, then the accumulate rounded, over the first `taps` samples of every K-sample
+ * row in tap order.  No reference has this mode; with the folded planner tables and taps == K it is
+ * orc_channelize_cs16 (tests/test_cs16_oracle.py). */
+void orc_channelize_cs16_table(const int16_t *iq, int nout, int K, int taps, int nch, const float *wf, float *dm)
+{
+	for (int m = 0; m < nout; m++) {
+		const int16_t *p = iq + (size_t)m * K * 2;
+		for (int ch = 0; ch < nch; ch++) {
+			const float *w = wf + (size_t)ch * 2 * taps;
+			float dr = 0, di = 0;
+			for (int ind = 0; ind < taps; ind++) {
+				float a = (float)p[2 * ind], b = (float)p[2 * ind + 1];
+				float c = w[2 * ind], d = w[2 * ind + 1];
+				float pr = a * c - b * d, pi = a * d + b * c;
+				dr = dr + pr;
+				di = di + pi;
+			}
+			dm[(size_t)ch * nout + m] = hypotf(dr, di);
+		}
+	}
+}
+
 /* ------------------------------------------------------------------ frame sync (acars.c) */
 
 #define SYN 0x16

@@ -89,6 +89,9 @@ void orc_channelize_real(const float *x, int nout, int K, int nch,
 void orc_cs16_build_osc(int variant, unsigned freq_hz, unsigned fc, int K, float *osc /*2K*/); /* soapy.c:159-162, sdrplay.c:133-137 */
 void orc_channelize_cs16(int variant, const int16_t *iq /*interleaved I,Q*/, int nout, int K, int nch,
                          const float *osc /*nch x 2K*/, float *dm /*nch x nout*/);          /* soapy.c:232-254, sdrplay.c:215-236 */
+/* a CS16 context with the caller's table (no reference implementation): plain D += v*w over the first `taps` samples */
+void orc_channelize_cs16_table(const int16_t *iq, int nout, int K, int taps, int nch,
+                               const float *wf /*nch x 2*taps*/, float *dm /*nch x nout*/);
 
 /* demod + framing (msk.c, acars.c) */
 void orc_chan_init(orc_chan_t *c, int chn);                           /* msk.c:30-51, acars.c:230-234 */

@@ -94,6 +94,35 @@ def assert_emission_order(got, model):
             assert m.pos == p, (s, t[0], m.pos, p)
 
 
+def ragged_sizes(K: int, total: int, max_submit: int, seed: int):
+    """Submit lengths in samples that cover `total`: below one row, a few rows, one block and 37 rows more (a pipeline
+    block and generic tail rows in one submit), an odd count, a couple of rows and one, then random lengths."""
+    rng = np.random.default_rng(seed)
+    sizes, pos = [], 0
+    for n in [K // 3 + 1, 5 * K + 7, 1061 * K + 13, 3, 2 * K + 1]:
+        sizes.append(min(n, total - pos, max_submit))
+        pos += sizes[-1]
+    while pos < total:
+        sizes.append(min(int(rng.integers(1, 1500 * K)), total - pos, max_submit))
+        pos += sizes[-1]
+    return [n for n in sizes if n]
+
+
+def stream_envelope(ctx, submit, data: np.ndarray, sizes):
+    """Feed data (nstreams, nsamples[, 2]) to a streaming context through `submit` in the given lengths and read each
+    submit's envelope right after it: (concatenated envelope (nstreams, nout, nch), drained messages)."""
+    pieces, msgs, pos = [], [], 0
+    for n in sizes:
+        m = submit(np.ascontiguousarray(data[:, pos:pos + n]))
+        pos += n
+        ctx.sync()
+        msgs += ctx.drain()
+        if m:
+            pieces.append(ctx.read_dm(m))
+    assert pos == data.shape[1]
+    return np.concatenate(pieces, axis=1), msgs
+
+
 def bits_equal(a: np.ndarray, b: np.ndarray) -> bool:
     from refs import Digest
     if isinstance(b, Digest):

@@ -368,6 +368,7 @@ class OracleLib:
         L.orc_channelize_dft8_cs16.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
         L.orc_cs16_build_osc.argtypes = [C.c_int, C.c_uint, C.c_uint, C.c_int, C.c_void_p]
         L.orc_channelize_cs16.argtypes = [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]
+        L.orc_channelize_cs16_table.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]
         L.orc_chan_init.argtypes = [C.POINTER(OrcChan), C.c_int]
         L.orc_demod.argtypes = [C.POINTER(OrcChan), C.c_void_p, C.c_void_p, C.c_int, C.POINTER(OrcSink)]
         L.orc_block_fec.argtypes = [C.POINTER(Msg)]
@@ -508,6 +509,16 @@ class OracleLib:
         dm = np.empty((osc.shape[0], nout), dtype=np.float32)
         osc = np.ascontiguousarray(osc, dtype=np.float32)
         self.lib.orc_channelize_cs16(variant, iq.ctypes.data, nout, K, osc.shape[0], osc.ctypes.data, dm.ctypes.data)
+        return dm
+
+    def channelize_cs16_table(self, iq: np.ndarray, K: int, taps: int, wf: np.ndarray) -> np.ndarray:
+        """A CS16 context with the caller's table: |sum of the first `taps` (float)int16 samples x wf| per K-sample row."""
+        iq = np.ascontiguousarray(iq, dtype=np.int16).reshape(-1)
+        nout = iq.size // (2 * K)
+        dm = np.empty((wf.shape[0], nout), dtype=np.float32)
+        wf = np.ascontiguousarray(wf, dtype=np.float32)
+        assert wf.shape[1] == 2 * taps
+        self.lib.orc_channelize_cs16_table(iq.ctypes.data, nout, K, taps, wf.shape[0], wf.ctypes.data, dm.ctypes.data)
         return dm
 
     def new_chan(self, chn: int) -> OrcChan:

@@ -76,3 +76,33 @@ def test_cs16_folded_tables_equal_literal_arithmetic(oracle):
         scale = np.float32(1 / 32768) if variant == 0 else np.float32(0.25)
         plain = oracle.channelize_cs16(2, iq, K, osc * scale)      # plain D += v*w ; |D|
         assert bits_equal(lit, plain), variant
+
+
+@pytest.mark.parametrize("K", [160, 36])
+def test_cs16_caller_table_restatement(oracle, K):
+    """orc_channelize_cs16_table (a CS16 context with acb_set_wf's table) is the literal arithmetic of both front-ends
+    when handed their folded planner tables, and at taps < K the same sum over the first `taps` samples: equal to a K-tap
+    table zero-padded past `taps` (x*0 = +-0 leaves D and |D| alone) and within rounding of a float64 sum."""
+    fm = FREQS if K == 160 else (131.525, 131.550, 131.600)
+    fd, _, fc = oracle.plan(K, fm)
+    iq = np.random.default_rng(K).integers(-32768, 32768, size=(48 * K, 2), dtype=np.int16)
+    iq[:K] = 32767
+    iq[K:2 * K] = -32768
+    for variant in (0, 1):
+        osc = oracle.cs16_osc(variant, K, fd, fc)
+        folded = api.build_wf_cs16(variant, K, fd, fc)
+        assert bits_equal(oracle.channelize_cs16_table(iq, K, K, folded), oracle.channelize_cs16(variant, iq, K, osc)), variant
+    rng = np.random.default_rng(K + 1)
+    x = iq.astype(np.float64).reshape(-1, K, 2)
+    x = x[..., 0] + 1j * x[..., 1]
+    for taps in (1, 5, K - 3):
+        wf = (rng.standard_normal((len(fm), 2 * taps)) * 1e-4).astype(np.float32)
+        got = oracle.channelize_cs16_table(iq, K, taps, wf)
+        padded = np.zeros((len(fm), 2 * K), dtype=np.float32)
+        padded[:, :2 * taps] = wf
+        assert bits_equal(got, oracle.channelize_cs16(2, iq, K, padded)), taps
+        w = wf[:, 0::2].astype(np.float64) + 1j * wf[:, 1::2]
+        d64 = x[:, :taps] @ w.T
+        mass = np.abs(x[:, :taps]) @ np.abs(w).T
+        assert (np.abs(got.T - np.abs(d64)) <= 2 * (taps + 4) * 2.0 ** -24 * mass).all(), taps
+        assert got.any()
