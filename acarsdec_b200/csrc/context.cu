@@ -87,7 +87,7 @@ struct acb_ctx {
 	cudaEvent_t ev_copied[2], ev_consumed[2];
 	bool buf_used[2];
 	int next_buf;
-	float *d_wf4;                /* [stream][grp][K][8] float4 (c, d, -d, c) */
+	float *d_wf4;                /* [stream][grp][K][8] float2 (c, d), every input kind */
 	bool fast;                   /* ACB_FLAG_FAST_CHANNELIZER and a shape k_channelize_dft takes */
 	bool fold8;                  /* fast form: fold the row in half first (8-way split, K/8 MACs per channel) */
 	int demod_lanes;             /* lanes per channel in k_demod: 8 for small contexts, else 4 */
@@ -308,7 +308,7 @@ extern "C" int acb_create(const acb_config_t *cfg, acb_ctx_t **out)
 		CU(cudaEventCreateWithFlags(&c->ev_consumed[i], cudaEventDisableTiming));
 	}
 	if (c->real_input) CU(cudaEventCreateWithFlags(&c->ev_real_copied, cudaEventDisableTiming));
-	const size_t wf_floats = (size_t)cfg->nstreams * c->ngrp * c->taps_pad * CH_GROUP * (c->in_kind == IN_KIND_F32REAL ? 2 : 4);
+	const size_t wf_floats = (size_t)cfg->nstreams * c->ngrp * c->taps_pad * CH_GROUP * 2;
 	CU(cudaMalloc(&c->d_wf4, wf_floats * sizeof(float)));
 	CU(cudaMemsetAsync(c->d_wf4, 0, wf_floats * sizeof(float), c->s_copy));
 	CU(cudaStreamSynchronize(c->s_copy));
@@ -431,15 +431,13 @@ extern "C" int acb_set_wf(acb_ctx_t *c, int stream, const float *wf, int nch)
 	if (stream < 0 || stream >= c->cfg.nstreams || nch != c->cfg.nch) return fail(ACB_ERR_ARG, "stream/nch mismatch");
 	if (int r = ctx_use(c)) return r;
 	const int T = c->taps, TP = c->taps_pad;      /* taps beyond T keep zero weights: D + (+0) = D */
-	const int W = c->in_kind == IN_KIND_F32REAL ? 2 : 4;
-	std::vector<float> t((size_t)c->ngrp * TP * CH_GROUP * W, 0.0f);
+	std::vector<float> t((size_t)c->ngrp * TP * CH_GROUP * 2, 0.0f);     /* (c, d) for every input kind */
 	for (int ch = 0; ch < nch; ch++) {
 		const int g = ch / CH_GROUP, cc = ch % CH_GROUP;
 		for (int ind = 0; ind < T; ind++) {
-			const float re = wf[((size_t)ch * T + ind) * 2], im = wf[((size_t)ch * T + ind) * 2 + 1];
-			float *o = &t[(((size_t)g * TP + ind) * CH_GROUP + cc) * W];
-			o[0] = re; o[1] = im;
-			if (W == 4) { o[2] = -im; o[3] = re; }            /* (c, d, -d, c): see cmac() */
+			float *o = &t[(((size_t)g * TP + ind) * CH_GROUP + cc) * 2];
+			o[0] = wf[((size_t)ch * T + ind) * 2];
+			o[1] = wf[((size_t)ch * T + ind) * 2 + 1];
 		}
 	}
 	if (int r = sync_streams(c)) return r;

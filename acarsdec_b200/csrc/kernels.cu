@@ -6,8 +6,8 @@
  *                     rx_callback air.c:291-341; soapy.c:232-254, sdrplay.c:215-236).  FP32-issue bound by the
  *                     reference's rounding sequence: every complex MAC is 4 rounded products
  *                     and 4 rounded sums in tap order, no FMA contraction — reproduced exactly
- *                     (packed FMUL2/FADD2 where ptxas keeps them unfused) so dm is bit-identical
- *                     to the strict-IEEE build of the reference.
+ *                     (IQ: two rows packed per FFMA2(x, w, -0) / FADD2, see cmac2) so dm is
+ *                     bit-identical to the strict-IEEE build of the reference.
  *      k_channelize_dft   : opt-in fast form of the u8 path (ACB_FLAG_FAST_CHANNELIZER): the same bins as a
  *                     shared 4-point DFT across the row quarters + K/4 MACs per channel; HBM-bound
  *                     (bulk copies, packed FFMA2); messages identical, envelope within tolerance.
@@ -44,29 +44,37 @@ int upload_matched_filter(const float *h, cudaStream_t stream);
  * K1: channelizer
  * ---------------------------------------------------------------------------------------- */
 
-/* (float)u8 - 127.37f  (rtl.c:338-339).  The byte is planted in the mantissa of 2^23, the
+/* (float)u8 - 127.37f  (rtl.c:338-339) for sample `pair` of word wa (row A) and of word wb (row B),
+ * row-packed: re = (I_A, I_B), im = (Q_A, Q_B).  The byte is planted in the mantissa of 2^23, the
  * 2^23 removed (exact), then 127.37f subtracted — also exact: the result is a multiple of
  * 2^-17 below 2^7, so the reference's single rounding rounds nothing either. */
-__device__ __forceinline__ float2 cvt_iq(unsigned w, int pair)
+__device__ __forceinline__ void cvt_iq(unsigned wa, unsigned wb, int pair, float2 &re, float2 &im)
 {
-	float2 x;
-	x.x = __uint_as_float(__byte_perm(w, 0x4B000000u, pair ? 0x7542 : 0x7540));
-	x.y = __uint_as_float(__byte_perm(w, 0x4B000000u, pair ? 0x7543 : 0x7541));
-	x = __fadd2_rn(x, make_float2(-8388608.0f, -8388608.0f));
-	return __fadd2_rn(x, make_float2(-127.37f, -127.37f));
+	re = make_float2(__uint_as_float(__byte_perm(wa, 0x4B000000u, pair ? 0x7542 : 0x7540)),
+	                 __uint_as_float(__byte_perm(wb, 0x4B000000u, pair ? 0x7542 : 0x7540)));
+	im = make_float2(__uint_as_float(__byte_perm(wa, 0x4B000000u, pair ? 0x7543 : 0x7541)),
+	                 __uint_as_float(__byte_perm(wb, 0x4B000000u, pair ? 0x7543 : 0x7541)));
+	re = __fadd2_rn(__fadd2_rn(re, make_float2(-8388608.0f, -8388608.0f)), make_float2(-127.37f, -127.37f));
+	im = __fadd2_rn(__fadd2_rn(im, make_float2(-8388608.0f, -8388608.0f)), make_float2(-127.37f, -127.37f));
 }
 
 /* D += (a + jb) * (c + jd) with the reference's rounding: products rounded, (ac - bd) and
- * (ad + bc) rounded, then the accumulate rounded (rtl.c:351).  w = (c, d, -d, c).
- * Instruction shape: 2 FMUL2 + 2 FADD + 1 FADD2.  The middle sums are deliberately scalar:
- * ptxas 12.9 contracts mul.rn.f32x2 feeding add.rn.f32x2 into FFMA2 even under -fmad=false
- * (checked in SASS), which would skip the product rounding; it leaves FMUL2 -> FADD alone. */
-__device__ __forceinline__ void cmac(float2 &acc, float a, float b, const float4 w)
+ * (ad + bc) rounded, then the accumulate rounded (rtl.c:351) — for two output rows at once,
+ * row-packed: a = (a_A, a_B), b = (b_A, b_B), Dre = (Dre_A, Dre_B), Dim = (Dim_A, Dim_B); the
+ * table entry (c, d) rides the packed ops' scalar operand.
+ * Instruction shape: 4 FFMA2 + 4 FADD2 for the two rows, i.e. 4 packed instructions per complex MAC.
+ * Every product is FFMA2(x, w, nz) with nz = -0.0f: rn(x*w + (-0)) = rn(x*w) for every finite
+ * x*w, signed zeros included, and an FFMA2 cannot be fused into the FADD2 that consumes it.  nz
+ * must be a run-time value (a kernel argument): ptxas turns an FFMA2 with a literal -0 addend
+ * back into FMUL2, and contracts mul.rn.f32x2 feeding add.rn.f32x2 into FFMA2 even under
+ * -fmad=false, which would skip a product rounding.  tests/test_sass_exact.py checks the SASS. */
+__device__ __forceinline__ void cmac2(float2 &dre, float2 &dim, const float2 a, const float2 b, float c, float d, float nz)
 {
-	const float2 p1 = __fmul2_rn(make_float2(a, a), make_float2(w.x, w.y));
-	const float2 p2 = __fmul2_rn(make_float2(b, b), make_float2(w.z, w.w));
-	const float2 t = make_float2(__fadd_rn(p1.x, p2.x), __fadd_rn(p1.y, p2.y));
-	acc = __fadd2_rn(acc, t);
+	const float2 z = make_float2(nz, nz), cc = make_float2(c, c), dd = make_float2(d, d);
+	const float2 ac = __ffma2_rn(a, cc, z), bd = __ffma2_rn(b, dd, z);
+	const float2 ad = __ffma2_rn(a, dd, z), bc = __ffma2_rn(b, cc, z);
+	dre = __fadd2_rn(dre, __fadd2_rn(ac, make_float2(-bd.x, -bd.y)));
+	dim = __fadd2_rn(dim, __fadd2_rn(ad, bc));
 }
 
 /* cabsf (rtl.c:353): glibc hypotf is (float)sqrt((double)x*x + (double)y*y) for finite input */
@@ -86,14 +94,14 @@ __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wai
 
 /* ------------------------------------------------------------------------------------------
  * K1 pipeline.  One CTA = one 1024-output block x one group of 8 channels; 128 threads, two
- * output rows per thread (rows t and t+128 of a 256-row tile) so every broadcast table load
- * feeds two complex MACs; the K taps are walked in chunks of 5 sixteen-byte units per row
+ * output rows per thread (rows t and t+128 of a 256-row tile) so every broadcast 16-byte table load
+ * (two channels' (c, d)) feeds four complex MACs; the K taps are walked in chunks of 5 sixteen-byte units per row
  * (5 is odd: the strided LDS.128 row reads are conflict free without padding) staged by
  * cp.async into a 2-deep ring together with the matching slice of the table, so the copy of
  * chunk i+1 runs under the arithmetic of chunk i.  Any K that keeps rows 16-byte aligned, up to
- * ACB_MAXK.  MODE: u8 IQ with table entries (c, d, -d, c) (rtl.c:334-354); float32 real samples,
- * D += wf[i]*S, entries (c, d) (air.c:314-333); CS16 IQ, same complex MAC as u8 on (float)int16
- * (soapy.c:239-242 with the /32768.0 folded into the table, sdrplay.c:218-222).
+ * ACB_MAXK.  Table entries are (c, d) for every MODE: u8 IQ (rtl.c:334-354), one LDS.128 serving
+ * two channels of cmac2; float32 real samples, D += wf[i]*S (air.c:314-333); CS16 IQ, same complex
+ * MAC as u8 on (float)int16 (soapy.c:239-242 with the /32768.0 folded into the table, sdrplay.c:218-222).
  * ---------------------------------------------------------------------------------------- */
 
 constexpr int C2_ROWS = 256;
@@ -109,22 +117,23 @@ template <int MODE> struct C2 {
 	static constexpr int STAGES = 2;                             /* cp.async ring depth */
 	static constexpr int TAP_BYTES = MODE == IN_U8IQ ? 2 : 4;    /* input bytes per tap */
 	static constexpr int TAPS_PER_UNIT = 16 / TAP_BYTES;
-	static constexpr int W_BYTES = MODE == IN_F32REAL ? 8 : 16;  /* table bytes per (tap, channel) */
+	static constexpr int W_BYTES = 8;                            /* table bytes per (tap, channel): (c, d) */
 	static constexpr int CHUNK_TAPS = UNITS * TAPS_PER_UNIT;
 	static constexpr int TILE_BYTES = C2_ROWS * ROW_UNITS * 16;
 	static constexpr int WF_BYTES = CHUNK_TAPS * CH_GROUP * W_BYTES;
 	static constexpr int STAGE_BYTES = TILE_BYTES + WF_BYTES;
 };
 
-/* (float)int16 for both halves of a CS16 sample (soapy.c:239-240, sdrplay.c:218-219): x ^ 0x8000
- * planted in the mantissa of 2^23, then 2^23 + 2^15 removed — exact */
-__device__ __forceinline__ float2 cvt_cs16(unsigned w)
+/* (float)int16 for both halves of a CS16 sample (soapy.c:239-240, sdrplay.c:218-219) of row A (word wa)
+ * and row B (word wb), row-packed like cvt_iq: x ^ 0x8000 planted in the mantissa of 2^23, then
+ * 2^23 + 2^15 removed — exact */
+__device__ __forceinline__ void cvt_cs16(unsigned wa, unsigned wb, float2 &re, float2 &im)
 {
-	const unsigned v = w ^ 0x80008000u;
-	float2 x;
-	x.x = __uint_as_float(__byte_perm(v, 0x4B000000u, 0x7410));
-	x.y = __uint_as_float(__byte_perm(v, 0x4B000000u, 0x7432));
-	return __fadd2_rn(x, make_float2(-8421376.0f, -8421376.0f));
+	const unsigned va = wa ^ 0x80008000u, vb = wb ^ 0x80008000u;
+	re = make_float2(__uint_as_float(__byte_perm(va, 0x4B000000u, 0x7410)), __uint_as_float(__byte_perm(vb, 0x4B000000u, 0x7410)));
+	im = make_float2(__uint_as_float(__byte_perm(va, 0x4B000000u, 0x7432)), __uint_as_float(__byte_perm(vb, 0x4B000000u, 0x7432)));
+	re = __fadd2_rn(re, make_float2(-8421376.0f, -8421376.0f));
+	im = __fadd2_rn(im, make_float2(-8421376.0f, -8421376.0f));
 }
 
 /* air.c:317-318: D += wf[i] * S — (c*S, d*S) rounded, then the accumulate rounded.  Scalar
@@ -137,8 +146,9 @@ __device__ __forceinline__ void rmac(float2 &acc, float sv, const float2 w)
 template <int MODE>
 __global__ void __launch_bounds__(CH_TILE)
 k_channelize(const uint8_t *__restrict__ in, size_t stream_stride, const uint8_t *__restrict__ wf,
-              float *__restrict__ dm, int K, int taps, int nch, int ngrp, size_t nsamp)
+              float *__restrict__ dm, int K, int taps, int nch, int ngrp, size_t nsamp, float nz)
 {
+	/* nz: -0.0f, the addend of cmac2's product FFMA2s (a kernel argument on purpose, see cmac2) */
 	using T = C2<MODE>;
 	extern __shared__ __align__(16) unsigned char smem[];
 	const int t = threadIdx.x;
@@ -181,9 +191,11 @@ k_channelize(const uint8_t *__restrict__ in, size_t stream_stride, const uint8_t
 			cp_async_commit();
 		};
 
-		float2 accA[CH_GROUP], accB[CH_GROUP];
+		/* float32 real: acc0 = row A (re, im), acc1 = row B (re, im).  IQ modes, row-packed for cmac2:
+		 * acc0 = re (row A, row B), acc1 = im (row A, row B). */
+		float2 acc0[CH_GROUP], acc1[CH_GROUP];
 #pragma unroll
-		for (int c = 0; c < CH_GROUP; c++) accA[c] = accB[c] = make_float2(0.f, 0.f);
+		for (int c = 0; c < CH_GROUP; c++) acc0[c] = acc1[c] = make_float2(0.f, 0.f);
 
 		/* prologue: STAGES-1 chunks in flight; every iteration commits exactly one group (possibly
 		 * empty) so that "all but the newest STAGES-1 groups" always means "chunk `step` landed" */
@@ -211,34 +223,26 @@ k_channelize(const uint8_t *__restrict__ in, size_t stream_stride, const uint8_t
 #pragma unroll
 						for (int c = 0; c < CH_GROUP; c++) {
 							const float2 w = wj[e * CH_GROUP + c];
-							rmac(accA[c], sa, w);
-							rmac(accB[c], sb, w);
-						}
-					}
-				} else if (MODE == IN_CS16IQ) {
-					const float4 *wj = reinterpret_cast<const float4 *>(st + T::TILE_BYTES) + (size_t)j * 4 * CH_GROUP;
-#pragma unroll
-					for (int e = 0; e < 4; e++) {
-						const float2 xa = cvt_cs16(wa[e]), xb = cvt_cs16(wb[e]);
-#pragma unroll
-						for (int c = 0; c < CH_GROUP; c++) {
-							const float4 w = wj[e * CH_GROUP + c];
-							cmac(accA[c], xa.x, xa.y, w);
-							cmac(accB[c], xb.x, xb.y, w);
+							rmac(acc0[c], sa, w);
+							rmac(acc1[c], sb, w);
 						}
 					}
 				} else {
-					const float4 *wj = reinterpret_cast<const float4 *>(st + T::TILE_BYTES) + (size_t)j * 8 * CH_GROUP;
+					/* one float4 = the (c, d) entries of channels 2i and 2i+1 */
+					constexpr int SPW = MODE == IN_CS16IQ ? 1 : 2;       /* complex samples per 32-bit word */
+					const float4 *wj = reinterpret_cast<const float4 *>(st + T::TILE_BYTES) + (size_t)j * 4 * SPW * CH_GROUP / 2;
 #pragma unroll
 					for (int e = 0; e < 4; e++) {
 #pragma unroll
-						for (int h = 0; h < 2; h++) {
-							const float2 xa = cvt_iq(wa[e], h), xb = cvt_iq(wb[e], h);
+						for (int h = 0; h < SPW; h++) {
+							float2 re, im;
+							if (MODE == IN_CS16IQ) cvt_cs16(wa[e], wb[e], re, im);
+							else cvt_iq(wa[e], wb[e], h, re, im);
 #pragma unroll
-							for (int c = 0; c < CH_GROUP; c++) {
-								const float4 w = wj[(2 * e + h) * CH_GROUP + c];
-								cmac(accA[c], xa.x, xa.y, w);
-								cmac(accB[c], xb.x, xb.y, w);
+							for (int c = 0; c < CH_GROUP; c += 2) {
+								const float4 w = wj[((SPW * e + h) * CH_GROUP + c) / 2];
+								cmac2(acc0[c], acc1[c], re, im, w.x, w.y, nz);
+								cmac2(acc0[c + 1], acc1[c + 1], re, im, w.z, w.w, nz);
 							}
 						}
 					}
@@ -248,20 +252,24 @@ k_channelize(const uint8_t *__restrict__ in, size_t stream_stride, const uint8_t
 				const int nc = min(CH_GROUP, nch - g * CH_GROUP);
 #pragma unroll
 				for (int half = 0; half < 2; half++) {
-					float2 *acc = half ? accB : accA;
+					float2 d[CH_GROUP];                              /* (re, im) of this half's row */
+#pragma unroll
+					for (int c = 0; c < CH_GROUP; c++)
+						d[c] = MODE == IN_F32REAL ? (half ? acc1[c] : acc0[c])
+						                          : (half ? make_float2(acc0[c].y, acc1[c].y) : make_float2(acc0[c].x, acc1[c].x));
 					const size_t m = (size_t)blk * OUTBLK + (size_t)tile * C2_ROWS + t + half * CH_TILE;
 					float *o = dm + ((size_t)s * nsamp + m) * nch + g * CH_GROUP;
 					if (nc == CH_GROUP && (nch & 3) == 0) {
-						reinterpret_cast<float4 *>(o)[0] = make_float4(envelope(acc[0]), envelope(acc[1]), envelope(acc[2]), envelope(acc[3]));
-						reinterpret_cast<float4 *>(o)[1] = make_float4(envelope(acc[4]), envelope(acc[5]), envelope(acc[6]), envelope(acc[7]));
+						reinterpret_cast<float4 *>(o)[0] = make_float4(envelope(d[0]), envelope(d[1]), envelope(d[2]), envelope(d[3]));
+						reinterpret_cast<float4 *>(o)[1] = make_float4(envelope(d[4]), envelope(d[5]), envelope(d[6]), envelope(d[7]));
 					} else {
 #pragma unroll
 						for (int c = 0; c < CH_GROUP; c++)
-							if (c < nc) o[c] = envelope(acc[c]);
+							if (c < nc) o[c] = envelope(d[c]);
 					}
-#pragma unroll
-					for (int c = 0; c < CH_GROUP; c++) acc[c] = make_float2(0.f, 0.f);
 				}
+#pragma unroll
+				for (int c = 0; c < CH_GROUP; c++) acc0[c] = acc1[c] = make_float2(0.f, 0.f);
 			}
 			__syncthreads();                                         /* stage may be refilled by issue(step+2) */
 		}
@@ -408,7 +416,7 @@ static int launch_channelize_t(const void *in, size_t stream_stride, const void 
 	if (e != cudaSuccess) return (int)e;
 	dim3 grid(nblk, nstreams, ngrp);
 	k_channelize<MODE><<<grid, CH_TILE, smem, stream>>>(reinterpret_cast<const uint8_t *>(in), stream_stride,
-	                                                    reinterpret_cast<const uint8_t *>(wf), dm, K, taps, nch, ngrp, nsamp);
+	                                                    reinterpret_cast<const uint8_t *>(wf), dm, K, taps, nch, ngrp, nsamp, -0.0f);
 	return (int)cudaGetLastError();
 }
 
@@ -1312,9 +1320,9 @@ k_channelize_generic(const uint8_t *__restrict__ in, size_t stream_stride, const
 	const size_t m = row0 + gid / nch;
 	const int ch = (int)(gid % nch);
 	float dr = 0.f, di = 0.f;
+	const float2 *w = reinterpret_cast<const float2 *>(wf) + ((size_t)s * ngrp + ch / CH_GROUP) * taps * CH_GROUP + (ch % CH_GROUP);
 	if (MODE == IN_F32REAL) {
 		const float *p = reinterpret_cast<const float *>(in + (size_t)s * stream_stride) + m * K;
-		const float2 *w = reinterpret_cast<const float2 *>(wf) + ((size_t)s * ngrp + ch / CH_GROUP) * taps * CH_GROUP + (ch % CH_GROUP);
 		for (int i = 0; i < taps; i++) {
 			const float2 ww = w[(size_t)i * CH_GROUP];
 			dr = __fadd_rn(dr, __fmul_rn(ww.x, p[i]));
@@ -1322,21 +1330,19 @@ k_channelize_generic(const uint8_t *__restrict__ in, size_t stream_stride, const
 		}
 	} else if (MODE == IN_CS16IQ) {
 		const short *p = reinterpret_cast<const short *>(in + (size_t)s * stream_stride) + m * K * 2;
-		const float4 *w = reinterpret_cast<const float4 *>(wf) + ((size_t)s * ngrp + ch / CH_GROUP) * taps * CH_GROUP + (ch % CH_GROUP);
 		for (int ind = 0; ind < taps; ind++) {
 			const float a = (float)p[2 * ind], b = (float)p[2 * ind + 1];
-			const float4 ww = w[(size_t)ind * CH_GROUP];
-			dr = __fadd_rn(dr, __fadd_rn(__fmul_rn(a, ww.x), __fmul_rn(b, ww.z)));
-			di = __fadd_rn(di, __fadd_rn(__fmul_rn(a, ww.y), __fmul_rn(b, ww.w)));
+			const float2 ww = w[(size_t)ind * CH_GROUP];
+			dr = __fadd_rn(dr, __fsub_rn(__fmul_rn(a, ww.x), __fmul_rn(b, ww.y)));
+			di = __fadd_rn(di, __fadd_rn(__fmul_rn(a, ww.y), __fmul_rn(b, ww.x)));
 		}
 	} else {
 		const uint8_t *p = in + (size_t)s * stream_stride + m * K * 2;
-		const float4 *w = reinterpret_cast<const float4 *>(wf) + ((size_t)s * ngrp + ch / CH_GROUP) * taps * CH_GROUP + (ch % CH_GROUP);
 		for (int ind = 0; ind < taps; ind++) {
 			float a = __fadd_rn((float)p[2 * ind], -127.37f), b = __fadd_rn((float)p[2 * ind + 1], -127.37f);
-			float4 ww = w[(size_t)ind * CH_GROUP];
-			float pr = __fadd_rn(__fmul_rn(a, ww.x), __fmul_rn(b, ww.z));
-			float pi = __fadd_rn(__fmul_rn(a, ww.y), __fmul_rn(b, ww.w));
+			float2 ww = w[(size_t)ind * CH_GROUP];
+			float pr = __fsub_rn(__fmul_rn(a, ww.x), __fmul_rn(b, ww.y));
+			float pi = __fadd_rn(__fmul_rn(a, ww.y), __fmul_rn(b, ww.x));
 			dr = __fadd_rn(dr, pr);
 			di = __fadd_rn(di, pi);
 		}
